@@ -348,6 +348,30 @@ def timed_steps(torch, hp, steps, warmup, world, dist, use_graph):
     return e0.elapsed_time(e1)
 
 
+DUMP_BYTES = 48 << 20   # --dump-outputs: bytes of the per-graph outputs written (dH and db come on top)
+
+
+def dump_outputs(hp, steps, out_dir):
+    """--dump-outputs: what the last timed step handed back to its caller, as float32 DIR/<name>.npy: y [B,N,F] (the
+    last layer's, node-major memory) and, when training, dX [B,G,N], dH [F,1,K,G], db [F].  Where y and dX of the whole
+    batch exceed DUMP_BYTES, the same graphs (drawn with a fixed seed) are written on every run."""
+    torch, w = hp.torch, hp.w
+    i = (steps - 1) % hp.ring                        # ring slot of the last timed step
+    per_graph = dict(y=hp.y2[i] if hp.layers == 2 else hp.y[i])
+    whole = {}
+    if hp.train:
+        per_graph["dX"] = hp.dX[i]
+        whole = dict(dH=hp.dH.view(w["F"], 1, w["K"], w["G"]), db=hp.db)
+    B = w["B"]
+    n = min(B, DUMP_BYTES // sum(t[0].numel() * t.element_size() for t in per_graph.values()))
+    if n < B:
+        idx = torch.from_numpy(np.sort(np.random.default_rng(0).choice(B, n, replace=False))).to(hp.dev)
+        per_graph = {k: t.index_select(0, idx) for k, t in per_graph.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in list(per_graph.items()) + list(whole.items()):
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 def kernel_alone_ms(torch, hp, which, reps):
     """average duration of the dominant kernel launched back to back (graph of `ring` launches,
     rotating batches) — second-stage reductions switched off so only that kernel runs."""
@@ -872,7 +896,14 @@ def main():
     ap.add_argument("--nccl", action="store_true", help="N > 1: plain NCCL all-reduce instead of the fused peer exchange")
     ap.add_argument("--no-extra", action="store_true", help="skip the side measurements of the other configs")
     ap.add_argument("--cpu-budget", type=float, default=12.0, help="seconds of CPU baseline work")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last one to DIR/<name>.npy (float32; a fixed "
+                         "sample of the graphs where the batch is large) so that two builds can be compared")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     w = WORKLOADS[args.config]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -931,6 +962,8 @@ def main():
     ms_max = float(t.item())
     value = world * w["B"] * steps / (ms_max * 1e-3)
     clocks = sampler.stop() if rank == 0 else None   # sampled over warm-up + the timed region of the headline
+    if args.dump_outputs and rank == 0:
+        dump_outputs(hp, steps, args.dump_outputs)
 
     dpc = dp_check(torch, dist, hp, world) if (world > 1 and w["train"]) else None
 

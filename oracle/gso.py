@@ -5,9 +5,9 @@ Only ``tests/``, ``__graft_entry__.smoke()`` and ``bench.py``'s cpu_baseline /
 product path.
 
 Parity pin: ``tests/test_oracle_golden.py`` checks every function here against
-golden vectors produced by *executing the reference itself* in the build
-container (``oracle/make_golden.py``), and — when ``/root/reference`` is
-present — against the live reference.
+golden vectors produced by *executing the reference itself*
+(``oracle/make_golden.py``), and — when ``GFC_REFERENCE_ROOT`` names a checkout
+of the original project — against the live reference.
 
 Two builders exist upstream:
 

@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE ONLY — generate ``tests/golden/*.npz`` by EXECUTING THE
-REFERENCE ITSELF (only possible in the build container where /root/reference
-exists).  Re-run with ``python -m oracle.make_golden`` from the repo root.
+REFERENCE ITSELF (only possible with a checkout of the original project).  Re-run
+with ``GFC_REFERENCE_ROOT=<checkout> python -m oracle.make_golden`` from the repo root.
 
 Everything stored under "expected" comes out of reference code:
   * ``Scene.readADjMatrix``                             (scene.py:140-154)
@@ -439,7 +439,7 @@ def model_param_layout():
 
 
 if __name__ == "__main__":
-    assert ri.available(), "run in the build container (needs /root/reference)"
+    assert ri.available(), "set GFC_REFERENCE_ROOT to a checkout of the original project"
     os.makedirs(OUT, exist_ok=True)
     gso_goldens()
     filter_goldens()

@@ -2,6 +2,7 @@
 (utils/graphUtils/graphML.py:2369-2488) — names, shapes, init law, asserts, repr,
 state_dict compatibility — and the product refuses to run without CUDA."""
 import math
+import os
 
 import numpy as np
 import pytest
@@ -9,6 +10,10 @@ import torch
 
 import gnnfc
 from oracle import refimport
+
+from util import rel_err
+
+NO_REFERENCE = "runs the original project's code: set GFC_REFERENCE_ROOT to a checkout of it"
 
 
 def test_constructor_and_parameters():
@@ -55,20 +60,38 @@ def test_no_cpu_fallback():
         gnnfc.build_gso(torch.zeros(2, 4, 2), 2.0)
 
 
-@pytest.mark.skipif(not refimport.available(), reason="reference tree only exists in the build container")
-def test_state_dict_roundtrip_with_reference_layer():
-    gml = refimport.graphml()
-    torch.manual_seed(3)
-    ref = gml.GraphFilterBatch(16, 8, 3)
-    ours = gnnfc.GraphFilterBatch(16, 8, 3)
-    ours.load_state_dict(ref.state_dict())        # same keys / shapes
-    assert torch.equal(ours.weight, ref.weight) and torch.equal(ours.bias, ref.bias)
-    ref.load_state_dict(ours.state_dict())
-    # same init law under the same seed
-    torch.manual_seed(5); a = gml.GraphFilterBatch(16, 8, 3)
-    torch.manual_seed(5); b = gnnfc.GraphFilterBatch(16, 8, 3)
-    assert torch.equal(a.weight, b.weight) and torch.equal(a.bias, b.bias)
-    assert repr(a) == repr(b)
+# (golden, torch seed): the taps stored in these goldens are the reference layer's own draw right after
+# torch.manual_seed(seed) (oracle/make_golden.py)
+REF_INIT_GOLDENS = {
+    "GraphFilterBatch": (("filter_cfg1.npz", 0), ("filter_general_e2.npz", 1), ("filter_k1_nobias.npz", 2),
+                         ("filter_nin_lt_n.npz", 3), ("filter_cfg2_symnorm.npz", 4), ("filter_cyclic.npz", 5),
+                         ("filter_cfg4_n12.npz", 6), ("filter_relu.npz", 12)),
+    "GraphFilter": (("samegso_e2_nin.npz", 10), ("samegso_cfg2_f32.npz", 11)),
+    "GraphFilterBatchGSO": (("batchgso_cfg2_3d.npz", 20), ("batchgso_e2_4d.npz", 21)),
+}
+
+
+def _check_reference_init(golden_dir, name):
+    """the reference layer's parameters load into ours (same keys / shapes) and our init law draws exactly them"""
+    layers = []
+    for fname, seed in REF_INIT_GOLDENS[name]:
+        g = np.load(os.path.join(golden_dir, fname))
+        F, E, K, G = g["h"].shape
+        ref_sd = {"weight": torch.from_numpy(g["h"])}
+        if "b" in g:
+            ref_sd["bias"] = torch.from_numpy(g["b"])
+        torch.manual_seed(seed)
+        ours = getattr(gnnfc, name)(G, F, K, E, bias="b" in g)
+        assert list(ours.state_dict().keys()) == list(ref_sd.keys())
+        for k, v in ref_sd.items():
+            assert torch.equal(ours.state_dict()[k], v), (fname, k)
+        ours.load_state_dict(ref_sd)
+        layers.append((ours, g))
+    return layers
+
+
+def test_state_dict_roundtrip_with_reference_layer(golden_dir):
+    _check_reference_init(golden_dir, "GraphFilterBatch")
 
 
 def test_shard_range_partitions_batch():
@@ -118,11 +141,11 @@ def test_recording_relayout_matches_the_reference_loops():
     S = gnnfc.gso_batch_from_recording(graph_rows, nA)
     assert S.shape == (T, 1, nA, nA) and S.is_contiguous() and S.dtype == torch.float32
     assert np.array_equal(S[:, 0].numpy(), c3[:, 0].astype(np.float32))          # suhaas_agent.py:117
-    # the live reference class, when the reference tree is present (build container only)
+    # the live reference class, when a checkout of the original project is given (GFC_REFERENCE_ROOT)
     from oracle import refimport
     if refimport.available():
         import sys
-        sys.path.insert(0, refimport.REF_ROOT) if hasattr(refimport, "REF_ROOT") else sys.path.insert(0, "/root/reference")
+        sys.path.insert(0, refimport.REF_ROOT)
         try:
             from custom_dataset import RobotDataset
         finally:
@@ -171,28 +194,24 @@ def test_same_gso_and_batch_gso_layers_surface():
         g(torch.zeros(2, 4, 2))                     # batchLSIGF asserts the node count, no zero-padding (:2154)
 
 
-@pytest.mark.skipif(not refimport.available(), reason="reference tree only exists in the build container")
-def test_new_layers_match_the_live_reference_surface():
-    gml = refimport.graphml()
-    for name, args, S in (("GraphFilter", (6, 5, 3, 2), torch.rand(2, 4, 4)),
-                          ("GraphFilterBatchGSO", (6, 5, 3, 1), torch.rand(7, 4, 4))):
-        torch.manual_seed(9); ref = getattr(gml, name)(*args)
-        torch.manual_seed(9); ours = getattr(gnnfc, name)(*args)
-        assert list(ref.state_dict().keys()) == list(ours.state_dict().keys())
-        assert torch.equal(ref.weight, ours.weight) and torch.equal(ref.bias, ours.bias)      # same init law / stream
-        assert ref.extra_repr() == ours.extra_repr()
-        ref.addGSO(S); ours.addGSO(S)
-        assert ref.extra_repr() == ours.extra_repr() and ref.N == ours.N
-        ours.load_state_dict(ref.state_dict())
-    # the powers attribute
-    torch.manual_seed(1)
-    S = torch.rand(3, 2, 5, 5)
-    ref = gml.GraphFilterBatchGSO(4, 4, 4, 2); ours = gnnfc.GraphFilterBatchGSO(4, 4, 4, 2)
-    ref.addGSO(S); ours.addGSO(S)
-    assert torch.allclose(ref.SK, ours.SK, rtol=1e-6, atol=1e-7)
+def test_new_layers_match_the_live_reference_surface(golden_dir):
+    """same keys, init law and draw order as the reference's GraphFilter / GraphFilterBatchGSO, and the
+    reference's extra_repr once a GSO is stored (both recorded from the reference by oracle/make_golden.py)"""
+    for ours, g in _check_reference_init(golden_dir, "GraphFilter"):
+        ours.addGSO(torch.from_numpy(g["S"]))
+        assert ours.N == g["S"].shape[-1]
+    for ours, g in _check_reference_init(golden_dir, "GraphFilterBatchGSO"):
+        ours.addGSO(torch.from_numpy(g["S"]))
+        assert ours.extra_repr() == str(g["repr"]) and ours.N == g["S"].shape[-1]
+        # the powers attribute: contracted with x and the taps it gives the reference's fp32 output
+        z = torch.einsum("bgm,bekmn->bekgn", torch.from_numpy(g["x"]).double(), ours.SK.double())
+        y = torch.einsum("fekg,bekgn->bfn", torch.from_numpy(g["h"]).double(), z) + torch.from_numpy(g["b"]).double()
+        if int(g["leaky"]):
+            y = torch.nn.functional.leaky_relu(y, 0.01)
+        assert rel_err(y.numpy(), g["y"]) < 3e-6
 
 
-@pytest.mark.skipif(not refimport.available(), reason="reference tree only exists in the build container")
+@pytest.mark.skipif(not refimport.available(), reason=NO_REFERENCE)
 def test_reference_policy_constructs_with_the_dropin_layer():
     """a10: the UNMODIFIED reference model file (graphs/models/suhaas_model.py) executed with its
     ``import utils.graphUtils.graphML as gml`` resolving to gnnfc: the GFL stage is built from the drop-in layer
@@ -252,23 +271,22 @@ def test_recurrent_layers_surface():
     assert torch.equal(gnnfc.torchpermul(w, x, b), (x.permute(0, 2, 1) * w.permute(1, 0)).permute(0, 2, 1) + b)
 
 
-@pytest.mark.skipif(not refimport.available(), reason="reference tree only exists in the build container")
-def test_recurrent_layers_match_the_live_reference_surface():
-    gml = refimport.graphml()
-    for name in ("GraphFilterRNNBatch", "GraphFilterMoRNNBatch", "GraphFilterL2ShareBatch"):
-        torch.manual_seed(3); ref = getattr(gml, name)(6, 5, 5, 2)
-        torch.manual_seed(3); ours = getattr(gnnfc, name)(6, 5, 5, 2)
-        assert [(k, tuple(v.shape)) for k, v in ref.state_dict().items()] == \
-               [(k, tuple(v.shape)) for k, v in ours.state_dict().items()]
-        for k in ref.state_dict():
-            assert torch.equal(ref.state_dict()[k], ours.state_dict()[k]), k       # same init law and draw order
-        assert ref.extra_repr() == ours.extra_repr()
-        S = torch.rand(3, 1, 5, 5)
-        ref.addGSO(S); ours.addGSO(S)
-        assert ref.extra_repr() == ours.extra_repr() and ref.N == ours.N
-        ours.load_state_dict(ref.state_dict())
-    x, w, b = torch.rand(2, 4, 4), torch.rand(4, 4), torch.rand(4, 1)
-    assert torch.equal(gml.torchpermul(w, x, b), gnnfc.torchpermul(w, x, b))
+def test_recurrent_layers_match_the_live_reference_surface(golden_dir):
+    """the parameters of the reference's recurrent layers right after torch.manual_seed(seed), as recorded in the
+    recurrent goldens (p_*, registration order; oracle/make_golden.py): ours draws the same ones in the same order"""
+    for tag, name, seed in (("rnn_n8", "GraphFilterRNNBatch", 21), ("rnn_nin", "GraphFilterRNNBatch", 22),
+                            ("mornn_n16", "GraphFilterMoRNNBatch", 23), ("l2share_n16", "GraphFilterL2ShareBatch", 24)):
+        g = np.load(os.path.join(golden_dir, "recurrent_%s.npz" % tag))
+        G, H, F, K, N = (int(v) for v in g["dims"][:5])
+        ref_sd = {k[2:]: torch.from_numpy(g[k]) for k in g.files if k.startswith("p_")}
+        torch.manual_seed(seed)
+        ours = getattr(gnnfc, name)(G, H, F, K)
+        assert list(ours.state_dict().keys()) == list(ref_sd.keys())
+        for k, v in ref_sd.items():
+            assert torch.equal(ours.state_dict()[k], v), (tag, k)                  # same init law and draw order
+        ours.load_state_dict(ref_sd)
+        ours.addGSO(torch.from_numpy(g["S"]))
+        assert ours.N == N
 
 
 # --------------------------------------------------------------------------- #
@@ -314,7 +332,7 @@ def test_recording_loader_matches_the_reference_dataset_loops():
     assert len(ld3) == 3 and list(ld3)[-1]["data"].shape[0] == 3
 
 
-@pytest.mark.skipif(not refimport.available(), reason="reference tree only exists in the build container")
+@pytest.mark.skipif(not refimport.available(), reason=NO_REFERENCE)
 def test_recording_loader_matches_the_live_robot_dataset():
     import sys
     sys.path.insert(0, refimport.REF_ROOT)

@@ -1,6 +1,6 @@
 """CPU: pins the oracle restatement (oracle/) against golden vectors that were
 produced by EXECUTING THE REFERENCE (oracle/make_golden.py), and against the
-live reference when /root/reference is present (build container only)."""
+live reference when GFC_REFERENCE_ROOT names a checkout of the original project."""
 import glob
 import os
 
@@ -194,7 +194,8 @@ def test_algebraic_properties_of_oracle():
     assert rel_err(yp, y @ P) < 1e-12
 
 
-@pytest.mark.skipif(not refimport.available(), reason="reference tree only exists in the build container")
+@pytest.mark.skipif(not refimport.available(),
+                    reason="runs the original project's code: set GFC_REFERENCE_ROOT to a checkout of it")
 def test_oracle_matches_live_reference():
     import torch
     gml = refimport.graphml()
